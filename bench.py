@@ -2,7 +2,7 @@
 """bench.py -- BASELINE.json metric: utterances/sec, ECAPA-TDNN + Fbank-80, 3 s @ 16 kHz, waveform -> 192-d
 embedding (configs[1]: batch 256 x 3 s synthetic audio per GPU).
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl ours|reference] [--precision bf16x3|bf16]
+  python bench.py [--gpus N --steps K --warmup W] [--impl ours|reference] [--precision bf16x3|bf16] [--dump-outputs DIR]
 
 One "step" = one batch of 256 utterances through the whole hot path.
   value     device-resident waveforms -> embeddings on device, CUDA events around the K timed steps, LANES batches in
@@ -17,6 +17,10 @@ N > 1: one process per GPU (torchrun), each rank extracts its own 256-utterance 
 data-path collective); barrier + synchronize on both sides; elapsed = max over ranks.
 --impl reference: the reference's own CPU path is pure Python over paddle/paddleaudio, which cannot be installed
 here (no network); the timed stand-in is the oracle port on all host cores (kind = "port").
+--dump-outputs DIR: after the timed passes, rank 0 writes the embeddings of the LAST timed step as DIR/<name>.npy (float32):
+  embeddings.npy      [256, 192] from the device-resident pass behind `value`
+  e2e_embeddings.npy  [256, 192] from the end-to-end pass (PPVectorPredictor.extract_embeddings_stream)
+Inputs and weights are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -56,6 +60,19 @@ def algorithmic_flops_per_utt(T=FRAMES, F=80, C=512, scale=8, A=128, S=128, E=19
 def synth_wave(batch, seed):
     g = torch.Generator().manual_seed(seed)
     return (0.1 * torch.randn(batch, SAMPLES, generator=g)).clamp_(-1, 1)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write {name: array} as path/<name>.npy, float64 kept as float64 and everything else as float32 (64 MB at most in all)."""
+    arrays = {k: np.ascontiguousarray(a, dtype=np.float64 if a.dtype == np.float64 else np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs: {total} bytes > {DUMP_LIMIT_BYTES}"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -240,7 +257,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="bf16x3", choices=["bf16x3", "bf16"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the embeddings of the last timed step as DIR/<name>.npy (rank 0, float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the CPU port times a calibrated, machine-dependent sample size)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -313,6 +336,9 @@ def main():
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if rank == 0 else None
     assert torch.isfinite(last).all() and torch.equal(last, emb)  # the last batch of both passes is the same input: bitwise equal embeddings
+    outputs = {}
+    if args.dump_outputs and rank == 0:  # host copy outside the timed regions
+        outputs["embeddings"] = last.cpu().numpy()
     del last
 
     # ---- end to end through the public API (host buffers) -----------------------------------------------------
@@ -325,6 +351,9 @@ def main():
     barrier()
     e2e_s = time.perf_counter() - t0
     assert np.isfinite(out.numpy()).all()
+    if args.dump_outputs and rank == 0:
+        outputs["e2e_embeddings"] = out.numpy().copy()
+        dump_outputs(args.dump_outputs, outputs)
 
     times = torch.tensor([ms / 1000.0, e2e_s, ms_single / 1000.0], dtype=torch.float64, device=dev)
     if dist is not None:

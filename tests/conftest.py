@@ -22,6 +22,19 @@ def golden_dir():
 
 
 @pytest.fixture(scope="session")
+def ref_head():
+    """tests/golden/ref_head.npz with every classifier gradient dW_<tag> rebuilt from the span coefficients dWspan_<tag>
+    that tests/golden/make_ref_fixtures.py stores for it (dW = emb^T c[:-1] + W * c[-1])."""
+    import numpy as np
+    g = np.load(os.path.join(GOLDEN, "ref_head.npz"))
+    d = {k: g[k] for k in g.files}
+    for k in [k for k in d if k.startswith("dWspan_")]:
+        c = d.pop(k)
+        d["dW_" + k[len("dWspan_"):]] = d["emb"].T @ c[:-1] + d["W"][:, :c.shape[1]] * c[-1]
+    return d
+
+
+@pytest.fixture(scope="session")
 def cuda():
     import torch
     if not torch.cuda.is_available():

@@ -32,6 +32,18 @@ def read_wav_int16(path):
         return np.frombuffer(w.readframes(w.getnframes()), dtype=np.int16).copy()
 
 
+def savez_lzma(path, arrays):
+    """np.savez with LZMA-compressed members (np.load reads them as usual): the int16 PCM and float32 features pack ~9 % tighter
+    than with deflate, which keeps fbank_wavs.npz under 1 MB."""
+    import io
+    import zipfile
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for k, a in arrays.items():
+            buf = io.BytesIO()
+            np.lib.format.write_array(buf, np.asanyarray(a))
+            z.writestr(k + ".npy", buf.getvalue())
+
+
 def ta_fbank(x):
     import torchaudio.compliance.kaldi as K
     return K.fbank(torch.from_numpy(np.ascontiguousarray(x, dtype=np.float32))[None], sample_frequency=16000.0,
@@ -48,7 +60,7 @@ def main():
     s = read_wav_int16(f"{REF}/dataset/test_long.wav")[160000:160000 + 48000]
     d["long3s_pcm"] = s
     d["long3s_fbank"] = ta_fbank(s.astype(np.float32) / 32768.0)
-    np.savez_compressed(f"{OUT}/fbank_wavs.npz", **d)
+    savez_lzma(f"{OUT}/fbank_wavs.npz", d)
     print({k: v.shape for k, v in d.items()})
 
     # ---- synthetic batch (SURVEY.md §8d config 2 recipe, 4 utterances)

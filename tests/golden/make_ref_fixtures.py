@@ -6,9 +6,13 @@ tests/test_oracle_vs_reference.py on any machine.  The files hold reference OUTP
 re-derived from seeds by the consumer (oracle.make_*_weights and `feats()` below), so agreement also pins
 parameter names and shapes (set_state_dict refuses missing / extra / mis-shaped keys).
 
-Usage:  python tests/golden/make_ref_fixtures.py            (rewrites the fixtures)
+Usage:  python tests/golden/make_ref_fixtures.py            (rewrites the fixtures and ref_digests.json)
         python tests/golden/make_ref_fixtures.py --check    (recomputes and compares with the committed files)
+ref_digests.json records a SHA-256 of every array the reference's code computed; tests/test_oracle_vs_reference.py checks
+the committed fixtures against it without needing the reference.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -226,7 +230,23 @@ def head_fixture():
     crit = AAMLoss(margin=0.0, scale=32)
     crit.update(margin=0.25)
     d["update_0.25"] = np.array([crit.cos_m, crit.sin_m, crit.th, crit.mmm])
+    for k in [k for k in d if k.startswith("dW_")]:
+        d["dWspan_" + k[len("dW_"):]] = span_coefficients(d["emb"], d["W"], d.pop(k))
     return d
+
+
+def span_coefficients(emb, W, dW):
+    """Every head here is a function of the cosine logits, so column j of the classifier's gradient is
+    (I - w_j w_j^T / |w_j|^2) / |w_j| * sum_b dlogit_bj * x_b / |x_b|: it lies in the span of the B embedding rows and w_j.
+    Store those B + 1 coefficients per column instead of its D entries (the fixture stays under 1 MB); the tests rebuild
+    dW = emb^T c[:-1] + W * c[-1] (conftest.py, fixture `ref_head`), checked here against the reference's dW."""
+    B, S = emb.shape[0], dW.shape[1]
+    c = np.empty((B + 1, S))
+    for j in range(S):
+        c[:, j] = np.linalg.lstsq(np.concatenate([emb.T, W[:, j:j + 1]], axis=1), dW[:, j], rcond=None)[0]
+    err = np.abs(emb.T @ c[:-1] + W[:, :S] * c[-1] - dW).max() / np.abs(dW).max()
+    assert err < 1e-13, err
+    return c
 
 
 def train_fixture():
@@ -293,13 +313,22 @@ def sched_fixture():
 
 FIXTURES = {"ref_models.npz": models_fixture, "ref_head.npz": head_fixture, "ref_train.npz": train_fixture,
             "ref_sched.npz": sched_fixture}
+DIGESTS = os.path.join(HERE, "ref_digests.json")
+
+
+def array_digest(a):
+    """dtype, shape and SHA-256 of the bytes of one array (same recipe in tests/test_oracle_vs_reference.py)."""
+    a = np.ascontiguousarray(a)
+    return {"dtype": a.dtype.str, "shape": list(a.shape), "sha256": hashlib.sha256(a.tobytes()).hexdigest()}
 
 
 def main():
     check = "--check" in sys.argv
     bad = 0
+    digests = {}
     for fn, make in FIXTURES.items():
         d = make()
+        digests[fn] = {k: array_digest(d[k]) for k in sorted(d)}  # written with the fixtures; --check compares values instead
         path = os.path.join(HERE, fn)
         if check:
             old = np.load(path)
@@ -310,6 +339,11 @@ def main():
         else:
             np.savez_compressed(path, **d)
             print(f"wrote {fn}: {len(d)} arrays, {os.path.getsize(path)} bytes")
+    if not check:
+        with open(DIGESTS, "w") as f:
+            json.dump(digests, f, indent=1, sort_keys=True)
+            f.write("\n")
+        print(f"wrote {os.path.basename(DIGESTS)}")
     sys.exit(1 if bad else 0)
 
 

@@ -98,12 +98,12 @@ def test_aam_config_size_vs_autograd(cuda):
 
 
 @pytest.mark.parametrize("kind,margin,ls", [("AM", 0.2, 0.0), ("AM", 0.35, 0.1), ("ARM", 0.2, 0.0), ("ARM", 0.1, 0.1), ("CE", 0.0, 0.0), ("CE", 0.0, 0.1)])
-def test_other_softmax_heads_match_the_reference_code(cuda, golden_dir, kind, margin, ls):
+def test_other_softmax_heads_match_the_reference_code(cuda, ref_head, kind, margin, ls):
     """AMLoss / ARMLoss / CELoss (ppvector/loss/amloss.py, armloss.py, celoss.py) on the fused CUDA head against what the REFERENCE's
     own loss classes computed (tests/golden/ref_head.npz, made by tests/golden/make_ref_fixtures.py): loss and both gradients."""
     from ppvector.loss import AMLoss, ARMLoss, CELoss
     from ppvector.models.fc import SpeakerIdentification
-    g = np.load(f"{golden_dir}/ref_head.npz")
+    g = ref_head
     emb = torch.from_numpy(g["emb"]).float().to(cuda).requires_grad_(True)
     clf = SpeakerIdentification(input_dim=192, num_speakers=g["W"].shape[1]).to(cuda)
     with torch.no_grad():
@@ -121,13 +121,13 @@ def test_other_softmax_heads_match_the_reference_code(cuda, golden_dir, kind, ma
 
 
 @pytest.mark.parametrize("K,margin,ls,easy", [(3, 0.2, 0.0, False), (3, 0.3, 0.1, False), (2, 0.2, 0.0, True)])
-def test_subcenter_loss_matches_the_reference_code(cuda, golden_dir, K, margin, ls, easy):
+def test_subcenter_loss_matches_the_reference_code(cuda, ref_head, K, margin, ls, easy):
     """SubCenterLoss (ppvector/loss/subcenterloss.py:33-54; classifier with K sub-centres per class, fc.py:33) on the fused CUDA head against
     the REFERENCE's own class (tests/golden/ref_head.npz): a class's cosine is the max over its K adjacent columns, the AAM margin rule on top,
     and only the winning sub-centre column receives the class's gradient."""
     from ppvector.loss import SubCenterLoss
     from ppvector.models.fc import SpeakerIdentification
-    g = np.load(f"{golden_dir}/ref_head.npz")
+    g = ref_head
     Sk = 156 // K
     emb = torch.from_numpy(g["emb"]).float().to(cuda).requires_grad_(True)
     clf = SpeakerIdentification(input_dim=192, num_speakers=Sk, K=K).to(cuda)
@@ -145,12 +145,12 @@ def test_subcenter_loss_matches_the_reference_code(cuda, golden_dir, K, margin, 
 
 
 @pytest.mark.parametrize("mt,margin,lam,t", [("C", 0.2, 0.7, 3), ("A", 0.15, 0.7, 3), ("C", 0.3, 0.5, 2)])
-def test_sphereface2_matches_the_reference_code(cuda, golden_dir, mt, margin, lam, t):
+def test_sphereface2_matches_the_reference_code(cuda, ref_head, mt, margin, lam, t):
     """SphereFace2 (ppvector/loss/sphereface2.py:44-70: per-entry binary logistic loss over g(z) = 2 ((z+1)/2)^t - 1, margin types 'C' and 'A')
     on the fused CUDA head against the REFERENCE's own class (tests/golden/ref_head.npz): loss and both gradients."""
     from ppvector.loss import SphereFace2
     from ppvector.models.fc import SpeakerIdentification
-    g = np.load(f"{golden_dir}/ref_head.npz")
+    g = ref_head
     emb = torch.from_numpy(g["emb"]).float().to(cuda).requires_grad_(True)
     clf = SpeakerIdentification(input_dim=192, num_speakers=g["W"].shape[1]).to(cuda)
     with torch.no_grad():
